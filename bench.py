@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the Chebyshev filtering hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 metric  = cheby_op filtered-vertices/sec = N * Nsig * order / t
 workload, 1 GPU : BASELINE configs[1] -- Sensor-type 2-D k-NN graph, N = 1e6, k = 10,
@@ -28,6 +28,10 @@ cpu_baseline: the unmodified reference (baseline/_ref; the oracle port if absent
           a bounded sample of the same workload.
 --impl reference: the unmodified reference's CPU path on up to 64 host processes
           (one signal column each; the reference is single-threaded by construction).
+--dump-outputs DIR: after the timed steps, what the last one returned, (Nscales, vertices,
+          signals) float32, as DIR/y.npy (DIR/y_rank<r>.npy on N > 1 GPUs); above DUMP_BYTES
+          in all, the rows of a fixed, seeded sample of vertices.  Graph and signals are
+          seeded, so two builds given the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -80,7 +84,14 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--cpu-columns", type=int, default=4)
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed under DIR (see above)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of --impl ours")
+    return args
 
 
 # ------------------------------------------------------------------ workload
@@ -356,6 +367,21 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------- our arm
+DUMP_BYTES = 48 << 20
+
+
+def dump_output(torch, path, name, y, max_bytes):
+    """y (..., vertices, signals) -> path/name.npy as computed; over max_bytes, the rows of
+    a fixed sample of vertices (seed 0: the same rows for the same vertex count)."""
+    n = y.shape[-2]
+    row_bytes = y.numel() // n * y.element_size()
+    if n * row_bytes > max_bytes:
+        rows = np.sort(np.random.default_rng(0).choice(n, max_bytes // row_bytes, replace=False))
+        y = y.index_select(y.dim() - 2, torch.from_numpy(rows).to(y.device))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, name + ".npy"), y.cpu().numpy())
+
+
 def build_graph(gsp, wl):
     """The workload's graph through the Graph API: adjacency, Laplacian and lmax on the device."""
     if wl["graph"] == "grid2d":
@@ -628,6 +654,9 @@ def run_ours(args):
     clocks.__exit__()
     t_dev = allmax(start.elapsed_time(stop) / 1e3)
     value = n_global * nsig * order * args.steps / t_dev
+    if args.dump_outputs:
+        dump_output(torch, args.dump_outputs, "y" if world == 1 else "y_rank%d" % rank, y_dev,
+                    DUMP_BYTES // world)
 
     # ---- end to end through the public API with host buffers
     e2e = None

@@ -31,10 +31,22 @@ def _stamp():
     return h.hexdigest()
 
 
+def _up_to_date():
+    stamp_file = os.path.join(OUT_DIR, "stamp.txt")
+    if not (os.path.exists(LIB) and os.path.exists(stamp_file)):
+        return False
+    with open(stamp_file) as fh:
+        return fh.read().strip() == _stamp()
+
+
 def build(force=False, verbose=False):
     """Build (if the sources changed) and return the path of the library.  One process at a
     time (flock on _lib/.lock: torchrun starts one process per GPU on the same tree); objects
-    and the library are written under temporary names and renamed into place."""
+    and the library are written under temporary names and renamed into place.  A library
+    built from the current sources is returned without writing anything, so that a built
+    tree can be used read-only."""
+    if not force and _up_to_date():
+        return LIB
     import fcntl
     os.makedirs(OUT_DIR, exist_ok=True)
     with open(os.path.join(OUT_DIR, ".lock"), "w") as lock:
@@ -46,11 +58,10 @@ def build(force=False, verbose=False):
 
 
 def _build_locked(force, verbose):
+    if not force and _up_to_date():
+        return LIB
     stamp_file = os.path.join(OUT_DIR, "stamp.txt")
     stamp = _stamp()
-    if not force and os.path.exists(LIB) and os.path.exists(stamp_file):
-        if open(stamp_file).read().strip() == stamp:
-            return LIB
     nvcc = _nvcc()
     objs = []
     procs = []
