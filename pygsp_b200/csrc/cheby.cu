@@ -21,25 +21,10 @@
 // gathers its packet of x_cur[col] -- a 16*G-byte contiguous, fully coalesced
 // request per neighbour -- and accumulates in registers.  The accumulation
 // order is the stored CSR order, i.e. the order scipy uses.
+#include <type_traits>
 #include "common.cuh"
-#include "gspb200.h"
 
 namespace gsp {
-
-int cheby_step_tiled_f32(bool first, int64_t rb, int64_t re, int64_t nnz, const int32_t* indptr,
-                         const int32_t* indices, const float* vals, const float* x_cur,
-                         const float* x_old, float* x_new, float* r, int64_t r_rows, int nsig,
-                         int nscales, const double* ck, const double* c0, double alpha, double beta,
-                         double gamma, const gsp_tile_plan& plan, const gsp_halo_fusion* halo,
-                         int64_t* rows_done, cudaStream_t st, bool add_source = false,
-                         bool reverse = false, const int64_t* out_perm = nullptr);
-int cheby_step_tiled_halo_f32(bool first, int64_t n, int64_t nnz, const int32_t* indptr,
-                              const int32_t* indices, const float* vals, const float* x_cur,
-                              const float* x_old, float* x_new, float* r, int64_t r_rows, int nsig,
-                              int nscales, const double* ck, const double* c0, double alpha,
-                              double beta, double gamma, const gsp_tile_plan& plan,
-                              const gsp_halo_fusion& halo, int64_t* rows_done, cudaStream_t st,
-                              bool add_source, bool reverse, const int64_t* out_perm);
 
 static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
@@ -268,38 +253,77 @@ int cheby_step(bool first, int64_t rb, int64_t re, const int32_t* indptr,
 }
 
 template <typename T>
-static int cheby_step_planned(const gsp_tile_plan* plan, int64_t nnz, bool first, int64_t rb,
-                              int64_t re, const int32_t* indptr, const int32_t* indices,
-                              const T* vals, const T* x_cur, const T* x_old, T* x_new, T* r,
-                              int64_t r_rows, int nsig, int nscales, const double* ck,
-                              const double* c0, double alpha, double beta, double gamma,
-                              cudaStream_t st, bool add_source = false, bool reverse = false) {
-  return cheby_step<T>(first, rb, re, indptr, indices, vals, x_cur, x_old, x_new, r, r_rows, nsig,
-                       nscales, ck, c0, alpha, beta, gamma, st, add_source);
+int run_step(const gsp_tile_plan* plan, const gsp_halo_fusion* halo, const Step<T>& s, int64_t rb,
+             int64_t re, int64_t nnz, const int32_t* indptr, const int32_t* indices, const T* vals,
+             int64_t r_rows, int nsig, cudaStream_t st, const int64_t* out_perm) {
+  const bool tiled = std::is_same<T, float>::value && plan && plan->rows_per_tile > 0 &&
+                     rb % 4 == 0 && s.nscales <= kMaxScales && aligned16(indptr) &&
+                     aligned16(indices) && aligned16(vals) && aligned16(s.x_cur) &&
+                     aligned16(s.x_new) && aligned16(s.r) && (s.first || aligned16(s.x_old));
+  if (halo && !tiled)
+    return fail(GSP_ERR_UNSUPPORTED, "fused halo step needs the tiled kernel (%s)", "plan");
+  int64_t done = rb;
+  if constexpr (std::is_same<T, float>::value) {
+    if (tiled) {
+      const int64_t R = plan->rows_per_tile;
+      const int64_t tiles = (re - rb) / R;
+      int64_t front = 0;
+      if (halo) {
+        // Two launches on one stream.  (1) The boundary ("front") tiles with the halo-capable
+        // instantiation: tiles whose rows read halo columns wait for the neighbours' flags, rows
+        // some neighbour needs are pushed into its halo, and the step is published once both sets
+        // are done.  (2) The interior tiles with the plain instantiation.  One kernel for both was
+        // 1.6 x slower per step: the boundary code's registers spilled inside the interior
+        // tiles' gather loop (ptxas, 60-register cap).  The front launch is a few dozen tiles
+        // (~10 us) and publishes before the interior runs.
+        GSP_REQUIRE(rb == 0, "fused halo push needs the whole row block in one launch");
+        GSP_REQUIRE(halo->n_wait <= 32, "at most 32 neighbours");
+        GSP_REQUIRE(halo->n_push_rows >= 0 && halo->n_boundary_rows >= 0, "negative row counts");
+        gsp_halo_fusion h = *halo;
+        h.n_wait_tiles = ceil_div(h.n_boundary_rows, R);
+        h.n_push_tiles = h.publish ? ceil_div(std::max(h.n_push_rows, h.n_boundary_rows), R) : 0;
+        front = std::max(h.n_wait_tiles, h.n_push_tiles);
+        GSP_REQUIRE(front <= tiles, "boundary rows must lie inside the full tiles");
+        if (front > 0) {
+          Step<float> f = s;
+          f.reverse = false;
+          int rc = cheby_step_tiled_f32(f, 0, front, &h, front, nnz, indptr, indices, vals, r_rows,
+                                        nsig, *plan, st, out_perm);
+          if (rc != GSP_OK) return rc;
+        }
+      }
+      int rc = cheby_step_tiled_f32(s, rb + front * R, tiles - front, nullptr, 0, nnz, indptr,
+                                    indices, vals, r_rows, nsig, *plan, st, out_perm);
+      if (rc != GSP_OK) return rc;
+      done = rb + tiles * R;
+    }
+  }
+  return cheby_step<T>(s.first, done, re, indptr, indices, vals, s.x_cur, s.x_old, s.x_new, s.r,
+                       r_rows, nsig, s.nscales, s.ck, s.c0, s.alpha, s.beta, s.gamma, st,
+                       s.add_source, out_perm);
 }
 
-// float32 with a tile plan: TMA-tiled kernel on the full tiles of [rb, re), the
-// row-group kernel on the remaining (< rows_per_tile) rows.
-template <>
-int cheby_step_planned<float>(const gsp_tile_plan* plan, int64_t nnz, bool first, int64_t rb,
-                              int64_t re, const int32_t* indptr, const int32_t* indices,
-                              const float* vals, const float* x_cur, const float* x_old,
-                              float* x_new, float* r, int64_t r_rows, int nsig, int nscales,
-                              const double* ck, const double* c0, double alpha, double beta,
-                              double gamma, cudaStream_t st, bool add_source, bool reverse) {
-  const bool tiled = plan && plan->rows_per_tile > 0 && rb % 4 == 0 && nscales <= kMaxScales &&
-                     aligned16(indptr) && aligned16(indices) && aligned16(vals) &&
-                     aligned16(x_cur) && aligned16(x_new) && aligned16(r) &&
-                     (first || aligned16(x_old));
-  int64_t done = 0;
-  if (tiled) {
-    int rc = cheby_step_tiled_f32(first, rb, re, nnz, indptr, indices, vals, x_cur, x_old, x_new, r,
-                                  r_rows, nsig, nscales, ck, c0, alpha, beta, gamma, *plan, nullptr,
-                                  &done, st, add_source, reverse);
+template <typename T>
+int cheby_forward(double lmax, const double* c, int nscales, int m, const T* x, T* r, T* t1, T* t2,
+                  const StepFn<T>& step) {
+  GSP_REQUIRE(nscales <= 1024, "at most 1024 filters per call");
+  double ck[1024], c0[1024];
+  for (int i = 0; i < nscales; ++i) c0[i] = c[int64_t(i) * m];
+  for (int k = 1; k < m; ++k) {
+    for (int i = 0; i < nscales; ++i) ck[i] = c[int64_t(i) * m + k];
+    // T_1 = (L x - a x)/a = (2/lmax) L x - x ; r_i = c_i0/2 T_0 + c_i1 T_1
+    // T_k = (4/lmax) L T_{k-1} - 2 T_{k-1} - T_{k-2}, written over T_{k-2} (row-local) for k >= 3
+    const bool first = k == 1;
+    T* dst = (k & 1) ? t1 : t2;
+    const T* cur = first ? x : ((k & 1) ? t2 : t1);
+    const T* old = first ? nullptr : (k == 2 ? x : dst);
+    // even k walks the tiles backwards: the lines of T_{k-1} and r that the previous
+    // step wrote last are still in L2 and are the first ones this step reads
+    int rc = step(k, {first, cur, old, dst, r, nscales, ck, c0, first ? 2.0 / lmax : 4.0 / lmax,
+                      first ? -1.0 : -2.0, first ? 0.0 : -1.0, false, (k & 1) == 0});
     if (rc != GSP_OK) return rc;
   }
-  return cheby_step<float>(first, rb + done, re, indptr, indices, vals, x_cur, x_old, x_new, r,
-                           r_rows, nsig, nscales, ck, c0, alpha, beta, gamma, st, add_source);
+  return GSP_OK;
 }
 
 // Full operator (approximations.py:58-114): K = m-1 fused steps on `stream`.
@@ -311,37 +335,11 @@ int cheby_op(int64_t n, int64_t nnz, const int32_t* indptr, const int32_t* indic
   GSP_REQUIRE(m >= 2, "The coefficients have an invalid shape");   // approximations.py:83-84
   GSP_REQUIRE(lmax > 0 && lmax == lmax, "lmax must be positive");
   if (n == 0) return GSP_OK;
-  double ck[1024], c0[1024];
-  GSP_REQUIRE(nscales <= 1024, "at most 1024 filters per call");
-  T* buf[2] = {work, work + n * int64_t(nsig)};
-  const T* t_old = x;
-  const T* t_cur = x;
-  for (int k = 1; k < m; ++k) {
-    for (int i = 0; i < nscales; ++i) {
-      ck[i] = coeffs[int64_t(i) * m + k];
-      c0[i] = coeffs[int64_t(i) * m];
-    }
-    int rc;
-    if (k == 1) {
-      // T_1 = (L x - a x)/a = (2/lmax) L x - x ; r_i = c_i0/2 T_0 + c_i1 T_1
-      rc = cheby_step_planned<T>(plan, nnz, true, 0, n, indptr, indices, vals, x, nullptr, buf[0],
-                                 r, n, nsig, nscales, ck, c0, 2.0 / lmax, -1.0, 0.0, st);
-      t_cur = buf[0];
-    } else {
-      // T_k = (4/lmax) L T_{k-1} - 2 T_{k-1} - T_{k-2}, written over T_{k-2}
-      // (row-local) except for k == 2 where T_0 is the caller's input.
-      T* dst = (k == 2) ? buf[1] : const_cast<T*>(t_old);
-      // odd steps walk the tiles backwards: the lines of T_{k-1} and r that the previous
-      // step wrote last are still in L2 and are the first ones this step reads
-      rc = cheby_step_planned<T>(plan, nnz, false, 0, n, indptr, indices, vals, t_cur, t_old, dst,
-                                 r, n, nsig, nscales, ck, c0, 4.0 / lmax, -2.0, -1.0, st, false,
-                                 (k & 1) == 0);
-      t_old = t_cur;
-      t_cur = dst;
-    }
-    if (rc != GSP_OK) return rc;
-  }
-  return GSP_OK;
+  return cheby_forward<T>(lmax, coeffs, nscales, m, x, r, work, work + n * int64_t(nsig),
+                          [&](int, const Step<T>& s) {
+                            return run_step<T>(plan, nullptr, s, 0, n, nnz, indptr, indices, vals,
+                                               n, nsig, st);
+                          });
 }
 
 // out = sum_i w[i] * src_i   (src: (nsrc, count) blocks) -- the top Clenshaw term S_K
@@ -368,49 +366,24 @@ __global__ void combine_sources(int64_t count, const T* __restrict__ src, int ns
 // the first step).  work holds 2*n*nsig elements.  Rounding differs from the forward
 // recurrence, the value does not (tests: same tolerance against the float64 oracle).
 template <typename T>
-int cheby_clenshaw(int64_t n, int64_t nnz, const int32_t* indptr, const int32_t* indices,
-                   const T* vals, double lmax, const double* c, int nsrc, int m, const T* src,
-                   int nsig, T* out, T* work, const gsp_tile_plan* plan, cudaStream_t st) {
-  GSP_REQUIRE(n >= 0 && nsig >= 1 && nsrc >= 1 && nsrc <= kMaxScales, "bad sizes");
-  GSP_REQUIRE(m >= 2, "The coefficients have an invalid shape");
-  GSP_REQUIRE(lmax > 0 && lmax == lmax, "lmax must be positive");
-  if (n == 0) return GSP_OK;
+int cheby_backward(double lmax, const double* c, int nsrc, int m, const T* src, T* out, T* b1,
+                   T* b2, const StepFn<T>& step) {
   const int K = m - 1;
   const double a2 = 4.0 / lmax;                  // 2 Lt = a2 L - 2 I
-  T* buf[2] = {work, work + n * int64_t(nsig)};
   T* xs = const_cast<T*>(src);                   // read-only source blocks
-  double ck[kMaxScales], zero[kMaxScales];
-  for (int i = 0; i < kMaxScales; ++i) zero[i] = 0;
-  auto coef_col = [&](int k, double scale) {
-    for (int i = 0; i < nsrc; ++i) ck[i] = scale * c[int64_t(i) * m + k];
-  };
-  const T* b_cur;
-  const T* b_old = nullptr;
-  int k_next;
+  double ck[kMaxScales], zero[kMaxScales] = {};
+  T* b_cur = b1;                                 // b_{k+1}
+  T* b_old = nullptr;                            // b_{k+2}
+  int s = 0, k_next = K - 1;
   if (nsrc == 1) {
-    if (K == 1) {                                // out = c0/2 x + c1 Lt x
-      return cheby_step_planned<T>(plan, nnz, true, 0, n, indptr, indices, vals, src, nullptr,
-                                   out, out, n, nsig, 0, zero, zero, c[1] * 2.0 / lmax,
-                                   0.5 * c[0] - c[1], 0.0, st);
-    }
+    if (K == 1)                                  // out = c0/2 x + c1 Lt x
+      return step(1, {true, src, nullptr, out, out, 0, zero, zero, c[1] * 2.0 / lmax,
+                      0.5 * c[0] - c[1], 0.0, false, false});
     // b_{K-1} = c_{K-1} x + 2 Lt (c_K x): b_K = c_K x is never materialised
-    int rc = cheby_step_planned<T>(plan, nnz, true, 0, n, indptr, indices, vals, src, nullptr,
-                                   buf[0], buf[0], n, nsig, 0, zero, zero, c[K] * a2,
-                                   c[K - 1] - 2.0 * c[K], 0.0, st);
+    int rc = step(++s, {true, src, nullptr, b1, b1, 0, zero, zero, c[K] * a2,
+                        c[K - 1] - 2.0 * c[K], 0.0, false, false});
     if (rc != GSP_OK) return rc;
-    b_cur = buf[0];
     k_next = K - 2;
-  } else {
-    // b_K = S_K by one combine pass
-    StepCoef<T> coef;
-    memset(&coef, 0, sizeof(coef));
-    for (int i = 0; i < nsrc; ++i) coef.ck[i] = T(c[int64_t(i) * m + K]);
-    const int64_t count = n * int64_t(nsig);
-    const int blocks = (int)std::min<int64_t>(ceil_div(count, 256), int64_t(sm_count()) * 16);
-    combine_sources<T><<<blocks, 256, 0, st>>>(count, src, nsrc, coef, buf[0]);
-    GSP_LAUNCH_CHECK("combine_sources");
-    b_cur = buf[0];
-    k_next = K - 1;
   }
   for (int k = k_next; k >= 0; --k) {
     const bool last = k == 0;
@@ -418,7 +391,7 @@ int cheby_clenshaw(int64_t n, int64_t nnz, const int32_t* indptr, const int32_t*
     // last  : out = (a2/2) L b_1 - b_1 - b_2 + S_0/2
     const double alpha = last ? 0.5 * a2 : a2, beta = last ? -1.0 : -2.0;
     double gamma = -1.0;
-    coef_col(k, last ? 0.5 : 1.0);
+    for (int i = 0; i < nsrc; ++i) ck[i] = (last ? 0.5 : 1.0) * c[int64_t(i) * m + k];
     const T* old = b_old;
     if (!old) {
       // no b_{k+2} buffer yet: it is c_K x (nsrc == 1, folded into the source term) or 0
@@ -426,15 +399,39 @@ int cheby_clenshaw(int64_t n, int64_t nnz, const int32_t* indptr, const int32_t*
       gamma = 0.0;
       old = b_cur;                                // any valid block, multiplied by 0
     }
-    T* dst = last ? out : (b_old ? const_cast<T*>(b_old) : buf[1]);
-    int rc = cheby_step_planned<T>(plan, nnz, false, 0, n, indptr, indices, vals, b_cur, old, dst,
-                                   xs, n, nsig, nsrc, ck, zero, alpha, beta, gamma, st, true,
-                               (k & 1) == 0);
+    T* dst = last ? out : (b_old ? b_old : b2);
+    int rc = step(++s, {false, b_cur, old, dst, xs, nsrc, ck, zero, alpha, beta, gamma, true,
+                        (k & 1) == 0});
     if (rc != GSP_OK) return rc;
     b_old = b_cur;
     b_cur = dst;
   }
   return GSP_OK;
+}
+
+template <typename T>
+int cheby_clenshaw(int64_t n, int64_t nnz, const int32_t* indptr, const int32_t* indices,
+                   const T* vals, double lmax, const double* c, int nsrc, int m, const T* src,
+                   int nsig, T* out, T* work, const gsp_tile_plan* plan, cudaStream_t st) {
+  GSP_REQUIRE(n >= 0 && nsig >= 1 && nsrc >= 1 && nsrc <= kMaxScales, "bad sizes");
+  GSP_REQUIRE(m >= 2, "The coefficients have an invalid shape");
+  GSP_REQUIRE(lmax > 0 && lmax == lmax, "lmax must be positive");
+  if (n == 0) return GSP_OK;
+  if (nsrc > 1) {
+    // b_K = S_K by one combine pass
+    StepCoef<T> coef;
+    memset(&coef, 0, sizeof(coef));
+    for (int i = 0; i < nsrc; ++i) coef.ck[i] = T(c[int64_t(i) * m + m - 1]);
+    const int64_t count = n * int64_t(nsig);
+    const int blocks = (int)std::min<int64_t>(ceil_div(count, 256), int64_t(sm_count()) * 16);
+    combine_sources<T><<<blocks, 256, 0, st>>>(count, src, nsrc, coef, work);
+    GSP_LAUNCH_CHECK("combine_sources");
+  }
+  return cheby_backward<T>(lmax, c, nsrc, m, src, out, work, work + n * int64_t(nsig),
+                           [&](int, const Step<T>& s) {
+                             return run_step<T>(plan, nullptr, s, 0, n, nnz, indptr, indices,
+                                                vals, n, nsig, st);
+                           });
 }
 
 // y = A x for a block of vectors (no recurrence, no r): used by Lanczos and
@@ -448,14 +445,21 @@ int spmm_plain(int64_t n, const int32_t* indptr, const int32_t* indices, const T
                        &none, 1.0, 0.0, 0.0, st);
 }
 
-template int cheby_step<float>(bool, int64_t, int64_t, const int32_t*, const int32_t*,
-                               const float*, const float*, const float*, float*, float*,
-                               int64_t, int, int, const double*, const double*, double,
-                               double, double, cudaStream_t, bool, const int64_t*);
-template int cheby_step<double>(bool, int64_t, int64_t, const int32_t*, const int32_t*,
-                                const double*, const double*, const double*, double*, double*,
-                                int64_t, int, int, const double*, const double*, double,
-                                double, double, cudaStream_t, bool, const int64_t*);
+#define GSP_INSTANTIATE(T)                                                                      \
+  template int cheby_step<T>(bool, int64_t, int64_t, const int32_t*, const int32_t*, const T*,  \
+                             const T*, const T*, T*, T*, int64_t, int, int, const double*,      \
+                             const double*, double, double, double, cudaStream_t, bool,         \
+                             const int64_t*);                                                   \
+  template int run_step<T>(const gsp_tile_plan*, const gsp_halo_fusion*, const Step<T>&,        \
+                           int64_t, int64_t, int64_t, const int32_t*, const int32_t*, const T*, \
+                           int64_t, int, cudaStream_t, const int64_t*);                         \
+  template int cheby_forward<T>(double, const double*, int, int, const T*, T*, T*, T*,          \
+                                const StepFn<T>&);                                              \
+  template int cheby_backward<T>(double, const double*, int, int, const T*, T*, T*, T*,         \
+                                 const StepFn<T>&);
+GSP_INSTANTIATE(float)
+GSP_INSTANTIATE(double)
+#undef GSP_INSTANTIATE
 
 }  // namespace gsp
 
@@ -478,10 +482,10 @@ extern "C" {
                            const double* c0_host, double alpha, double beta, double gamma,        \
                            const gsp_tile_plan* plan_host, void* stream) {                        \
     GSP_REQUIRE(nsig >= 1 && nsig <= (1 << 20), "nsig out of range");                             \
-    return gsp::cheby_step_planned<T>(plan_host, nnz, first != 0, row_begin, row_end, indptr,     \
-                                      indices, data, x_cur, x_old, x_new, r, r_rows, (int)nsig,   \
-                                      nscales, ck_host, c0_host, alpha, beta, gamma,              \
-                                      gsp::as_stream(stream));                                    \
+    const gsp::Step<T> s = {first != 0, x_cur, x_old, x_new, r, nscales, ck_host, c0_host,        \
+                            alpha, beta, gamma, false, false};                                    \
+    return gsp::run_step<T>(plan_host, nullptr, s, row_begin, row_end, nnz, indptr, indices,      \
+                            data, r_rows, (int)nsig, gsp::as_stream(stream));                     \
   }                                                                                               \
   int gsp_cheby_clenshaw_##SUF(int64_t n, int64_t nnz, const int32_t* indptr,                     \
                                const int32_t* indices, const T* data, double lmax,                \
@@ -512,16 +516,10 @@ int gsp_cheby_step_halo_f32(int first, int64_t n_rows, int64_t nnz, const int32_
   if (!(plan_host && plan_host->rows_per_tile > 0 && halo_host))
     return gsp::fail(GSP_ERR_UNSUPPORTED, "fused halo step needs a tile plan (%s)", "plan");
   GSP_REQUIRE(nscales <= gsp::kMaxScales, "too many filters for the fused step");
-  int64_t done = 0;
-  int rc = gsp::cheby_step_tiled_halo_f32(first != 0, n_rows, nnz, indptr, indices, data, x_cur,
-                                          x_old, x_new, r, r_rows, (int)nsig, nscales, ck_host,
-                                          c0_host, alpha, beta, gamma, *plan_host, *halo_host, &done,
-                                          gsp::as_stream(stream), false, reverse != 0, nullptr);
-  if (rc != GSP_OK) return rc;
-  // remainder rows (< rows_per_tile, interior by construction) with the row-group kernel
-  return gsp::cheby_step<float>(first != 0, done, n_rows, indptr, indices, data, x_cur, x_old,
-                                x_new, r, r_rows, (int)nsig, nscales, ck_host, c0_host, alpha,
-                                beta, gamma, gsp::as_stream(stream));
+  const gsp::Step<float> s = {first != 0, x_cur, x_old, x_new, r, nscales, ck_host, c0_host,
+                              alpha, beta, gamma, false, reverse != 0};
+  return gsp::run_step<float>(plan_host, halo_host, s, 0, n_rows, nnz, indptr, indices, data,
+                              r_rows, (int)nsig, gsp::as_stream(stream));
 }
 
 }  // extern "C"

@@ -660,63 +660,46 @@ static int launch_tiled_g(bool first, const TileArgs& a, bool halo, bool two, in
   return launch_tiled_gh<G, false, 1>(first, a, bps, st);
 }
 
-// Full tiles of rows [rb, re) of one step (rb % 4 == 0); reports the number of rows done.
-int cheby_step_tiled_f32(bool first, int64_t rb, int64_t re, int64_t nnz, const int32_t* indptr,
-                         const int32_t* indices, const float* vals, const float* x_cur,
-                         const float* x_old, float* x_new, float* r, int64_t r_rows, int nsig,
-                         int nscales, const double* ck, const double* c0, double alpha, double beta,
-                         double gamma, const gsp_tile_plan& plan, const gsp_halo_fusion* halo,
-                         int64_t* rows_done, cudaStream_t st, bool add_source, bool reverse,
+int cheby_step_tiled_f32(const Step<float>& s, int64_t rb, int64_t n_tiles,
+                         const gsp_halo_fusion* halo, int64_t n_front, int64_t nnz,
+                         const int32_t* indptr, const int32_t* indices, const float* vals,
+                         int64_t r_rows, int nsig, const gsp_tile_plan& plan, cudaStream_t st,
                          const int64_t* out_perm) {
+  const bool first = s.first;
   TileArgs a;
   a.out_perm = out_perm;
-  a.vec_direct = (!first && env_int("GSPB200_TILE_VDIR", add_source ? 1 : 0)) ? 1 : 0;
+  a.vec_direct = (!first && env_int("GSPB200_TILE_VDIR", s.add_source ? 1 : 0)) ? 1 : 0;
   a.keep_writes = env_int("GSPB200_TILE_REV", 1);
-  a.reverse = (reverse && a.keep_writes) ? 1 : 0;
-  a.add_source = add_source ? 1 : 0;
+  a.reverse = (s.reverse && a.keep_writes) ? 1 : 0;
+  a.add_source = s.add_source ? 1 : 0;
   a.l2_hint = env_int("GSPB200_TILE_HINT", 1);
-  a.n_front = 0;
-  GSP_REQUIRE(!add_source || (nscales >= 1 && !first), "add_source needs source blocks");
+  a.n_front = halo ? n_front : 0;
+  GSP_REQUIRE(!s.add_source || (s.nscales >= 1 && !first), "add_source needs source blocks");
   memset(&a.halo, 0, sizeof(a.halo));
-  const int64_t full_tiles = (re - rb) / plan.rows_per_tile;
   gsp_halo_fusion probe;                       // GSPB200_FORCE_HALO=1: run the halo-capable
   if (!halo && rb == 0 && env_int("GSPB200_FORCE_HALO", 0)) {   // variant with no neighbours
     memset(&probe, 0, sizeof(probe));          // (single-GPU A/B of the two instantiations)
     probe.n_owned = 0x7fffffff;
     halo = &probe;
   }
-  if (halo) {
-    a.halo = *halo;
-    const int R = plan.rows_per_tile;
-    GSP_REQUIRE(rb == 0, "fused halo push needs the whole row block in one launch");
-    GSP_REQUIRE(halo->n_wait <= 32, "at most 32 neighbours");
-    GSP_REQUIRE(halo->n_push_rows >= 0 && halo->n_boundary_rows >= 0, "negative row counts");
-    // tiles whose rows read halo columns wait for the neighbours' flags; the step is
-    // published once those AND the tiles that push rows are done (both sets are "front")
-    a.halo.n_wait_tiles = ceil_div(halo->n_boundary_rows, R);
-    a.halo.n_push_tiles =
-        halo->publish ? ceil_div(std::max(halo->n_push_rows, halo->n_boundary_rows), R) : 0;
-    a.n_front = std::max(a.halo.n_wait_tiles, a.halo.n_push_tiles);
-    GSP_REQUIRE(a.n_front <= full_tiles, "boundary rows must lie inside the full tiles");
-  }
+  if (halo) a.halo = *halo;
   a.row_begin = rb;
-  a.n_tiles = full_tiles;
-  *rows_done = a.n_tiles * plan.rows_per_tile;
+  a.n_tiles = n_tiles;
   if (a.n_tiles == 0) return GSP_OK;
   a.r_rows = r_rows;
   a.nnz = nnz;
   a.indptr = indptr; a.indices = indices; a.vals = vals;
-  a.x_cur = x_cur; a.x_old = x_old; a.x_new = x_new; a.r = r;
+  a.x_cur = s.x_cur; a.x_old = s.x_old; a.x_new = s.x_new; a.r = s.r;
   a.rows_per_tile = plan.rows_per_tile;
   a.slab_cap = plan.slab_capacity;
   a.stages = plan.stages;
   a.consumer_warps = plan.consumer_warps;
   a.nsig = nsig;
-  a.nscales = nscales;
-  a.alpha = float(alpha); a.beta = float(beta); a.gamma = float(gamma);
+  a.nscales = s.nscales;
+  a.alpha = float(s.alpha); a.beta = float(s.beta); a.gamma = float(s.gamma);
   for (int i = 0; i < kTiledMaxScales; ++i) {
-    a.ck[i] = i < nscales ? float(ck[i]) : 0.f;
-    a.half_c0[i] = (first && i < nscales) ? float(0.5 * c0[i]) : 0.f;
+    a.ck[i] = i < s.nscales ? float(s.ck[i]) : 0.f;
+    a.half_c0[i] = (first && i < s.nscales) ? float(0.5 * s.c0[i]) : 0.f;
   }
   const bool h = halo != nullptr;
   // two packets per lane (32 / 64 / 128 signals): a CSR read in shared memory serves twice
@@ -736,41 +719,6 @@ int cheby_step_tiled_f32(bool first, int64_t rb, int64_t re, int64_t nnz, const 
     case 128: return launch_tiled_g<32>(first, a, h, two, plan.blocks_per_sm, st);
   }
   return fail(GSP_ERR_UNSUPPORTED, "tiled kernel: nsig must be 8, 16, 32, 64 or 128 (%s)", "nsig");
-}
-
-// One step of the vertex-partitioned path on rows [0, n): two launches on one stream.
-// (1) The boundary ("front") tiles -- those holding rows that read halo columns or that some
-// neighbour needs -- with the halo-capable instantiation: wait for the neighbours' flags, coherent
-// gathers, peer stores of the new boundary rows, publish.  (2) All interior tiles with the plain
-// instantiation.  One kernel for both was 1.6 x slower per step (DESIGN.md section 5): under the
-// 60-register cap ptxas spilled the boundary code's state inside the interior gather loop.  The
-// front launch is a few dozen tiles (~10 us) and publishes before the interior tiles run, so the
-// neighbours' next front launch finds the flag set.  Reports the rows done (whole tiles).
-int cheby_step_tiled_halo_f32(bool first, int64_t n, int64_t nnz, const int32_t* indptr,
-                              const int32_t* indices, const float* vals, const float* x_cur,
-                              const float* x_old, float* x_new, float* r, int64_t r_rows, int nsig,
-                              int nscales, const double* ck, const double* c0, double alpha,
-                              double beta, double gamma, const gsp_tile_plan& plan,
-                              const gsp_halo_fusion& halo, int64_t* rows_done, cudaStream_t st,
-                              bool add_source, bool reverse, const int64_t* out_perm) {
-  const int64_t R = plan.rows_per_tile;
-  const int64_t front_rows =
-      ceil_div(std::max<int64_t>(halo.publish ? halo.n_push_rows : 0, halo.n_boundary_rows), R) * R;
-  GSP_REQUIRE(front_rows <= (n / R) * R, "boundary rows must lie inside the full tiles");
-  int64_t done_front = 0, done = 0;
-  if (front_rows > 0) {
-    int rc = cheby_step_tiled_f32(first, 0, front_rows, nnz, indptr, indices, vals, x_cur, x_old,
-                                  x_new, r, r_rows, nsig, nscales, ck, c0, alpha, beta, gamma, plan,
-                                  &halo, &done_front, st, add_source, false, out_perm);
-    if (rc != GSP_OK) return rc;
-    GSP_REQUIRE(done_front == front_rows, "front tiles must be whole tiles");
-  }
-  int rc = cheby_step_tiled_f32(first, front_rows, n, nnz, indptr, indices, vals, x_cur, x_old,
-                                x_new, r, r_rows, nsig, nscales, ck, c0, alpha, beta, gamma, plan,
-                                nullptr, &done, st, add_source, reverse, out_perm);
-  if (rc != GSP_OK) return rc;
-  *rows_done = front_rows + done;
-  return GSP_OK;
 }
 
 }  // namespace gsp

@@ -15,124 +15,8 @@
 #include <vector>
 #include <cstdio>
 #include "common.cuh"
-#include "gspb200.h"
 
 namespace gsp {
-
-int cheby_step_tiled_f32(bool first, int64_t rb, int64_t re, int64_t nnz, const int32_t* indptr,
-                         const int32_t* indices, const float* vals, const float* x_cur,
-                         const float* x_old, float* x_new, float* r, int64_t r_rows, int nsig,
-                         int nscales, const double* ck, const double* c0, double alpha, double beta,
-                         double gamma, const gsp_tile_plan& plan, const gsp_halo_fusion* halo,
-                         int64_t* rows_done, cudaStream_t st, bool add_source, bool reverse,
-                         const int64_t* out_perm);
-
-template <typename T> struct DistTraits;
-template <> struct DistTraits<float> {
-  static int push(const gsp_dist_plan* p, int64_t n_send, int b, uint64_t value, int64_t nsig,
-                  void* st) {
-    return gsp_halo_push_f32(n_send, p->src_row, p->dst_peer, p->dst_row,
-                             static_cast<const float*>(p->buf[b]),
-                             reinterpret_cast<float* const*>(p->peer_base[b]), nsig, p->peer_flags,
-                             p->n_neighbors, value, p->push_counter, st);
-  }
-};
-template <> struct DistTraits<double> {
-  static int push(const gsp_dist_plan* p, int64_t n_send, int b, uint64_t value, int64_t nsig,
-                  void* st) {
-    return gsp_halo_push_f64(n_send, p->src_row, p->dst_peer, p->dst_row,
-                             static_cast<const double*>(p->buf[b]),
-                             reinterpret_cast<double* const*>(p->peer_base[b]), nsig, p->peer_flags,
-                             p->n_neighbors, value, p->push_counter, st);
-  }
-};
-
-// One step on the whole local block.  Fused form (float32 + tile plan): wait, push and publish
-// happen inside the step kernel; otherwise wait kernel -> step -> push kernel.
-template <typename T>
-static int dist_step(const gsp_dist_plan* p, const gsp_tile_plan* tile, bool fused, bool first,
-                     const T* x_cur, const T* x_old, T* x_new, int new_buf, T* r, int64_t r_rows,
-                     int nsig, int nscales, const double* ck, const double* c0, double alpha,
-                     double beta, double gamma, bool add_source, bool reverse, uint64_t wait_value,
-                     uint64_t publish_value, bool publish, void* stream,
-                     const int64_t* out_perm = nullptr) {
-  cudaStream_t st = as_stream(stream);
-  const int64_t n = p->n_local;
-  if (fused) {
-    gsp_halo_fusion h;
-    memset(&h, 0, sizeof(h));
-    h.n_push_rows = publish ? p->n_push_rows : 0;
-    h.push_ptr = p->push_ptr;
-    h.push_peer = p->push_peer;
-    h.push_row = p->push_row;
-    h.peer_base = new_buf >= 0 ? p->peer_base[new_buf] : nullptr;
-    h.peer_flags = p->peer_flags;
-    h.push_counter = p->fused_counter;
-    h.wait_flags = p->flags;
-    h.wait_ids = p->neighbor_ids;
-    h.publish_value = publish_value;
-    h.wait_value = wait_value;
-    h.n_neighbors = p->n_neighbors;
-    h.n_wait = p->n_neighbors;
-    h.n_boundary_rows = p->n_boundary_rows;
-    h.n_owned = n;
-    h.publish = publish ? 1 : 0;
-    // Two launches on the same stream.  (1) The boundary ("front") tiles with the
-    // halo-capable instantiation: wait for the neighbours' flags, coherent gathers, peer
-    // stores of the new boundary rows, publish.  (2) All interior tiles with the plain
-    // instantiation.  One kernel for both was 1.6 x slower per step: the boundary code's
-    // registers spilled inside the interior tiles' gather loop (ptxas, 60-register cap);
-    // the front launch is a few dozen tiles (~10 us) and publishes before the interior runs.
-    const int R = tile->rows_per_tile;
-    const int64_t front_rows =
-        ceil_div(std::max<int64_t>(publish ? p->n_push_rows : 0, p->n_boundary_rows), (int64_t)R) * R;
-    int64_t done = 0, done_front = 0;
-    int rc = GSP_OK;
-    if (front_rows > 0) {
-      rc = cheby_step_tiled_f32(first, 0, front_rows, p->nnz, p->indptr, p->indices,
-                                reinterpret_cast<const float*>(p->data),
-                                reinterpret_cast<const float*>(x_cur),
-                                reinterpret_cast<const float*>(x_old),
-                                reinterpret_cast<float*>(x_new), reinterpret_cast<float*>(r), r_rows,
-                                nsig, nscales, ck, c0, alpha, beta, gamma, *tile, &h, &done_front, st,
-                                add_source, false, out_perm);
-      if (rc != GSP_OK) return rc;
-      GSP_REQUIRE(done_front == front_rows, "front tiles must be whole tiles");
-    }
-    rc = cheby_step_tiled_f32(first, front_rows, n, p->nnz, p->indptr, p->indices,
-                              reinterpret_cast<const float*>(p->data),
-                              reinterpret_cast<const float*>(x_cur),
-                              reinterpret_cast<const float*>(x_old), reinterpret_cast<float*>(x_new),
-                              reinterpret_cast<float*>(r), r_rows, nsig, nscales, ck, c0, alpha, beta,
-                              gamma, *tile, nullptr, &done, st, add_source, reverse, out_perm);
-    if (rc != GSP_OK) return rc;
-    done += front_rows;
-    // remainder rows (< rows_per_tile; interior by the fused-form condition)
-    return cheby_step<T>(first, done, n, p->indptr, p->indices, static_cast<const T*>(p->data), x_cur,
-                         x_old, x_new, r, r_rows, nsig, nscales, ck, c0, alpha, beta, gamma, st,
-                         add_source, out_perm);
-  }
-  int rc = gsp_halo_wait(p->flags, p->neighbor_ids, p->n_neighbors, wait_value, stream);
-  if (rc != GSP_OK) return rc;
-  int64_t done = 0;
-  if (std::is_same<T, float>::value && tile && tile->rows_per_tile > 0) {
-    // the TMA-tiled kernel without the fused exchange (the halo is complete: the wait kernel
-    // ran), then the row-group kernel on the < rows_per_tile remainder
-    rc = cheby_step_tiled_f32(first, 0, n, p->nnz, p->indptr, p->indices,
-                              reinterpret_cast<const float*>(p->data),
-                              reinterpret_cast<const float*>(x_cur),
-                              reinterpret_cast<const float*>(x_old), reinterpret_cast<float*>(x_new),
-                              reinterpret_cast<float*>(r), r_rows, nsig, nscales, ck, c0, alpha, beta,
-                              gamma, *tile, nullptr, &done, st, add_source, reverse, out_perm);
-    if (rc != GSP_OK) return rc;
-  }
-  rc = cheby_step<T>(first, done, n, p->indptr, p->indices, static_cast<const T*>(p->data), x_cur,
-                     x_old, x_new, r, r_rows, nsig, nscales, ck, c0, alpha, beta, gamma, st,
-                     add_source, out_perm);
-  if (rc != GSP_OK) return rc;
-  if (publish) return DistTraits<T>::push(p, p->n_send, new_buf, publish_value, nsig, stream);
-  return GSP_OK;
-}
 
 // GSPB200_DIST_TRACE=1: per-step CUDA-event times of one call on stderr (diagnosis; synchronises)
 struct StepTrace {
@@ -180,6 +64,7 @@ int cheby_op_dist(const gsp_dist_plan* p, const gsp_tile_plan* tile, double lmax
   const uint64_t base = *seq;
   *seq = base + uint64_t(m) + 2;
   T* buf[3] = {static_cast<T*>(p->buf[0]), static_cast<T*>(p->buf[1]), static_cast<T*>(p->buf[2])};
+  const T* data = static_cast<const T*>(p->data);
   const bool tiled = std::is_same<T, float>::value && tile && tile->rows_per_tile > 0;
   const bool fused =
       tiled && !p->separate_exchange && p->n_neighbors >= 1 && p->n_neighbors <= 32 &&
@@ -189,7 +74,7 @@ int cheby_op_dist(const gsp_dist_plan* p, const gsp_tile_plan* tile, double lmax
   StepTrace trace(st);
   trace.mark();
   // entry barrier, input block, halo of T_0
-  int rc = DistTraits<T>::push(p, 0, 0, base + 1, nsig, stream);
+  int rc = halo_push<T>(p, 0, 0, base + 1, nsig, st);
   if (rc != GSP_OK) return rc;
   rc = gsp_halo_wait(p->flags, p->neighbor_ids, p->n_neighbors, base + 1, stream);
   if (rc != GSP_OK) return rc;
@@ -200,74 +85,68 @@ int cheby_op_dist(const gsp_dist_plan* p, const gsp_tile_plan* tile, double lmax
   } else if (x && x != buf[0]) {
     GSP_CUDA(cudaMemcpyAsync(buf[0], x, sizeof(T) * size_t(n) * nsig, cudaMemcpyDeviceToDevice, st));
   }
-  rc = DistTraits<T>::push(p, p->n_send, 0, base + 2, nsig, stream);
+  rc = halo_push<T>(p, p->n_send, 0, base + 2, nsig, st);
   if (rc != GSP_OK) return rc;
   trace.mark();
 
-  double ck[16], c0[16], zero[16];
-  for (int i = 0; i < 16; ++i) zero[i] = 0;
-  if (!clenshaw) {
-    // forward recurrence, reference order (approximations.py:99-112).  With a row
-    // permutation the accumulators live in local order in stream-ordered scratch and are
-    // scattered to the caller's order at the end.
-    T* r_out = r;
-    if (perm && n > 0) {
-      GSP_CUDA(cudaMallocAsync((void**)&r, sizeof(T) * size_t(nscales) * n * nsig, st));
+  // Step s waits for the halo of x_cur (base + 1 + s) and, unless it is the last one, publishes
+  // the halo of x_new (base + 2 + s).  Fused form (float32 + tile plan): wait, push and publish
+  // happen inside the step kernel; otherwise wait kernel -> step -> push kernel.
+  const StepFn<T> step = [&](int s, const Step<T>& sp) {
+    const bool publish = s < K;
+    int b = 0;                          // state buffer x_new is (3: the caller's output)
+    while (b < 3 && buf[b] != sp.x_new) ++b;
+    const int64_t* out_perm = (clenshaw && s == K) ? perm : nullptr;
+    int rc;
+    if (fused) {
+      gsp_halo_fusion h;
+      memset(&h, 0, sizeof(h));
+      h.n_push_rows = publish ? p->n_push_rows : 0;
+      h.push_ptr = p->push_ptr;
+      h.push_peer = p->push_peer;
+      h.push_row = p->push_row;
+      h.peer_base = b < 3 ? p->peer_base[b] : nullptr;
+      h.peer_flags = p->peer_flags;
+      h.push_counter = p->fused_counter;
+      h.wait_flags = p->flags;
+      h.wait_ids = p->neighbor_ids;
+      h.publish_value = base + 2 + s;
+      h.wait_value = base + 1 + s;
+      h.n_neighbors = p->n_neighbors;
+      h.n_wait = p->n_neighbors;
+      h.n_boundary_rows = p->n_boundary_rows;
+      h.n_owned = n;
+      h.publish = publish ? 1 : 0;
+      rc = run_step<T>(tile, &h, sp, 0, n, p->nnz, p->indptr, p->indices, data, n, nsig, st,
+                       out_perm);
+    } else {
+      rc = gsp_halo_wait(p->flags, p->neighbor_ids, p->n_neighbors, base + 1 + s, stream);
+      if (rc == GSP_OK)
+        rc = run_step<T>(tile, nullptr, sp, 0, n, p->nnz, p->indptr, p->indices, data, n, nsig, st,
+                         out_perm);
+      if (rc == GSP_OK && publish) rc = halo_push<T>(p, p->n_send, b, base + 2 + s, nsig, st);
     }
-    int cur = 0, old = 1;
-    for (int k = 1; k <= K; ++k) {
-      for (int i = 0; i < nscales; ++i) {
-        ck[i] = c[int64_t(i) * m + k];
-        c0[i] = c[int64_t(i) * m];
-      }
-      const bool first = k == 1;
-      rc = dist_step<T>(p, tile, fused, first, buf[cur], first ? nullptr : buf[old], buf[old], old, r,
-                        n, nsig, nscales, ck, c0, first ? 2.0 / lmax : 4.0 / lmax,
-                        first ? -1.0 : -2.0, first ? 0.0 : -1.0, false, (k & 1) == 0,
-                        base + 1 + k, base + 2 + k, k < K, stream);
-      if (rc != GSP_OK) { if (r != r_out) cudaFreeAsync(r, st); return rc; }
-      trace.mark();
-      std::swap(cur, old);
-    }
-    if (r != r_out) {
-      for (int i = 0; i < nscales && rc == GSP_OK; ++i)
-        rc = move_rows<T>(true, n, perm, r + int64_t(i) * n * nsig, nsig, r_out + int64_t(i) * n * nsig,
-                          st);
-      cudaFreeAsync(r, st);
-    }
+    if (rc == GSP_OK) trace.mark();
     return rc;
+  };
+  // Clenshaw, single filter: buf[0] keeps x (the source), the b_k rotate through buf[1] and
+  // buf[2], the last step writes r
+  if (clenshaw) return cheby_backward<T>(lmax, c, 1, m, buf[0], r, buf[1], buf[2], step);
+  // forward recurrence, reference order, T_2 over T_0 in buf[0].  With a row permutation the
+  // accumulators live in local order in stream-ordered scratch and are scattered to the
+  // caller's order at the end.
+  T* r_out = r;
+  if (perm && n > 0) {
+    GSP_CUDA(cudaMallocAsync((void**)&r, sizeof(T) * size_t(nscales) * n * nsig, st));
   }
-  // Clenshaw, single filter (see cheby_clenshaw in cheby.cu): buf[0] keeps x (the source),
-  // b_{K-1} -> buf[1], b_{K-2} -> buf[2], b_{K-3} -> buf[1], ...; the last step writes r.
-  const double a2 = 4.0 / lmax;
-  rc = dist_step<T>(p, tile, fused, true, buf[0], nullptr, buf[1], 1, buf[1], n, nsig, 0, zero, zero,
-                    c[K] * a2, c[K - 1] - 2.0 * c[K], 0.0, false, false, base + 2, base + 3, true,
-                    stream);
-  if (rc != GSP_OK) return rc;
-  trace.mark();
-  int cur = 1, old = -1, step = 1;
-  for (int k = K - 2; k >= 0; --k) {
-    ++step;
-    const bool last = k == 0;
-    double gamma = -1.0;
-    ck[0] = (last ? 0.5 : 1.0) * c[k];
-    int old_buf = old;
-    if (old < 0) {                       // b_{K} = c_K x is folded into the source term
-      ck[0] -= c[K];
-      gamma = 0.0;
-      old_buf = cur;
-    }
-    const int dst = last ? -1 : (old >= 0 ? old : 2);
-    T* x_new = last ? r : buf[dst];
-    rc = dist_step<T>(p, tile, fused, false, buf[cur], buf[old_buf], x_new, dst, buf[0], n, nsig, 1,
-                      ck, zero, last ? 0.5 * a2 : a2, last ? -1.0 : -2.0, gamma, true, (k & 1) == 0,
-                      base + 1 + step, base + 2 + step, !last, stream, last ? perm : nullptr);
-    if (rc != GSP_OK) return rc;
-    trace.mark();
-    old = cur;
-    cur = dst;
+  rc = cheby_forward<T>(lmax, c, nscales, m, buf[0], r, buf[1], buf[0], step);
+  if (r != r_out) {
+    for (int i = 0; i < nscales && rc == GSP_OK; ++i)
+      rc = move_rows<T>(true, n, perm, r + int64_t(i) * n * nsig, nsig, r_out + int64_t(i) * n * nsig,
+                        st);
+    cudaFreeAsync(r, st);
   }
-  return GSP_OK;
+  return rc;
 }
 
 }  // namespace gsp

@@ -59,6 +59,32 @@ __global__ void halo_wait_kernel(const unsigned long long* flags, const int32_t*
   }
 }
 
+template <typename T>
+static int push_rows(int64_t n_send, const int64_t* src_row, const int32_t* dst_peer,
+                     const int64_t* dst_row, const T* src, T* const* peer_base, int64_t width,
+                     uint64_t* const* peer_flags, int n_neighbors, uint64_t value,
+                     uint32_t* done_counter, cudaStream_t st) {
+  const int64_t total = n_send * width;
+  const int blocks =
+      (int)std::max<int64_t>(1, std::min<int64_t>(ceil_div(total, 256), int64_t(sm_count()) * 4));
+  halo_push_kernel<T><<<blocks, 256, 0, st>>>(
+      n_send, src_row, dst_peer, dst_row, src, peer_base, width,
+      reinterpret_cast<unsigned long long* const*>(peer_flags), n_neighbors,
+      (unsigned long long)value, done_counter);
+  GSP_LAUNCH_CHECK("halo_push");
+  return GSP_OK;
+}
+
+template <typename T>
+int halo_push(const gsp_dist_plan* p, int64_t n_send, int b, uint64_t value, int64_t width,
+              cudaStream_t st) {
+  return push_rows<T>(n_send, p->src_row, p->dst_peer, p->dst_row, static_cast<const T*>(p->buf[b]),
+                      reinterpret_cast<T* const*>(p->peer_base[b]), width, p->peer_flags,
+                      p->n_neighbors, value, p->push_counter, st);
+}
+template int halo_push<float>(const gsp_dist_plan*, int64_t, int, uint64_t, int64_t, cudaStream_t);
+template int halo_push<double>(const gsp_dist_plan*, int64_t, int, uint64_t, int64_t, cudaStream_t);
+
 }  // namespace gsp
 
 extern "C" {
@@ -100,15 +126,9 @@ int gsp_ipc_free(void* dev_ptr) {
                           const int64_t* dst_row, const T* src, T* const* peer_base,             \
                           int64_t width, uint64_t* const* peer_flags, int n_neighbors,           \
                           uint64_t value, uint32_t* done_counter, void* stream) {                \
-    const int64_t total = n_send * width;                                                        \
-    const int blocks = (int)std::max<int64_t>(                                                   \
-        1, std::min<int64_t>(gsp::ceil_div(total, 256), int64_t(gsp::sm_count()) * 4));          \
-    gsp::halo_push_kernel<T><<<blocks, 256, 0, gsp::as_stream(stream)>>>(                        \
-        n_send, src_row, dst_peer, dst_row, src, peer_base, width,                               \
-        reinterpret_cast<unsigned long long* const*>(peer_flags), n_neighbors,                   \
-        (unsigned long long)value, done_counter);                                                \
-    GSP_LAUNCH_CHECK("halo_push");                                                               \
-    return GSP_OK;                                                                               \
+    return gsp::push_rows<T>(n_send, src_row, dst_peer, dst_row, src, peer_base, width,          \
+                             peer_flags, n_neighbors, value, done_counter,                       \
+                             gsp::as_stream(stream));                                            \
   }
 
 GSP_HALO_API(f32, float)
