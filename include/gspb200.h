@@ -382,6 +382,51 @@ int gsp_knn_to_csr_f64(int64_t n, int k, const int32_t* nn_idx, const double* nn
 GSPB200_DECLARE_GRAPH_API(f32, float)
 GSPB200_DECLARE_GRAPH_API(f64, double)
 
+/* ----------------------------------------------------------- differential operator ---
+ * D is the N x Ne incidence matrix of pygsp/graphs/difference.py (L = D D^T).  Edge k =
+ * (sources[k], targets[k]) with weight weights[k]; column k of D holds -v_s at the source and
+ * +v_t at the target, v = sqrt(w) (lap_type 0) or sqrt(w / dw) (lap_type 1), both divided by
+ * sqrt(2) when directed != 0; a self-loop's column is empty.  Every value is computed in double
+ * with correctly rounded operations and rounded once to T.  Two layouts of D:
+ *   edge-major   (d_*): SciPy's CSC arrays of D -- indptr (Ne + 1), row (vertex) indices, values;
+ *                       0 entries for a self-loop, 2 for any other edge, the smaller vertex first;
+ *   vertex-major (v_*): D as CSR (N x Ne), edge ids ascending within a row.
+ * gsp_edge_list_count / _fill_*  graph.py:1022-1029  get_edge_list(): every stored entry of W in
+ *     row-major order (directed != 0), else the upper triangle, diagonal included.  The count
+ *     writes edge_ptr (n + 1), whose last element is Ne; the fill writes int32 sources and
+ *     targets and the weights.
+ * gsp_diffop_count / _fill_*  difference.py compute_differential_operator().  The count writes
+ *     d_indptr (Ne + 1), whose last element is nnz(D); the fill writes d_indices / d_data and the
+ *     vertex-major layout (v_indptr has n + 1 entries).  dw is the weighted degree (double).
+ *     2 * Ne must fit int32 (else -1).
+ * gsp_grad_*  difference.py grad(): y (Ne, nsig) = D^T x, x (n, nsig), over the edge-major layout.
+ * gsp_div_*   difference.py div():  z (n, nsig) = D y, y (Ne, nsig), over the vertex-major layout.
+ *     Both start every output at +0.0 and add the products in stored order, multiply and add
+ *     rounded separately (no FMA): the result equals SciPy's D.T.dot(x) / D.dot(y) on the same D
+ *     bit for bit.
+ */
+int gsp_edge_list_count(int64_t n, const int32_t* indptr, const int32_t* indices, int directed,
+                        int32_t* edge_ptr, void* stream);
+int gsp_diffop_count(int64_t n_edges, const int32_t* sources, const int32_t* targets,
+                     int32_t* d_indptr, void* stream);
+
+#define GSPB200_DECLARE_DIFFOP_API(SUF, T)                                                       \
+  int gsp_edge_list_fill_##SUF(int64_t n, const int32_t* indptr, const int32_t* indices,         \
+                               const T* data, int directed, const int32_t* edge_ptr,            \
+                               int32_t* sources, int32_t* targets, T* weights, void* stream);   \
+  int gsp_diffop_fill_##SUF(int64_t n, int64_t n_edges, int64_t nnz, const int32_t* sources,     \
+                            const int32_t* targets, const T* weights, const double* dw,          \
+                            int lap_type, int directed, const int32_t* d_indptr,                 \
+                            int32_t* d_indices, T* d_data, int32_t* v_indptr,                    \
+                            int32_t* v_indices, T* v_data, void* stream);                        \
+  int gsp_grad_##SUF(int64_t n_edges, const int32_t* d_indptr, const int32_t* d_indices,         \
+                     const T* d_data, const T* x, int64_t nsig, T* y, void* stream);            \
+  int gsp_div_##SUF(int64_t n, const int32_t* v_indptr, const int32_t* v_indices,                \
+                    const T* v_data, const T* y, int64_t nsig, T* z, void* stream);
+
+GSPB200_DECLARE_DIFFOP_API(f32, float)
+GSPB200_DECLARE_DIFFOP_API(f64, double)
+
 #ifdef __cplusplus
 }
 #endif

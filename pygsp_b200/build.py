@@ -10,7 +10,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "_lib")
 LIB = os.path.join(OUT_DIR, "libgspb200.so")
-SOURCES = ["runtime.cu", "cheby.cu", "cheby_tiled.cu", "graph.cu", "lanczos.cu", "halo.cu", "generate.cu", "staging.cu", "dist.cu", "cg.cu"]
+SOURCES = ["runtime.cu", "cheby.cu", "cheby_tiled.cu", "graph.cu", "lanczos.cu", "halo.cu", "generate.cu", "staging.cu", "dist.cu", "cg.cu", "diffop.cu"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 
 

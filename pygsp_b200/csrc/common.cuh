@@ -131,6 +131,17 @@ template <typename T>
 int move_rows(bool scatter, int64_t rows, const int64_t* idx, const T* src, int64_t width, T* dst,
               cudaStream_t st);
 
+// indptr[1..n] holds row sizes on entry (indptr[0] = 0) and their inclusive scan on exit --
+// csrc/graph.cu, the scan of every count / fill pair
+int scan_rows(int32_t* indptr, int64_t n, cudaStream_t st);
+
+// Transpose of an n_rows x n_cols CSR as sorted CSR (t_indptr has n_cols + 1 entries); the
+// entries of a row of the result keep ascending column order -- csrc/graph.cu
+template <typename T>
+int csr_transpose(int64_t n_rows, int64_t n_cols, int64_t nnz, const int32_t* indptr,
+                  const int32_t* indices, const T* data, int32_t* t_indptr, int32_t* t_indices,
+                  T* t_data, cudaStream_t st);
+
 // ----- vector types: 16-byte packets of T --------------------------------
 template <typename T, int VEC> struct Pack;
 template <> struct Pack<float, 4> { typedef float4 type; };

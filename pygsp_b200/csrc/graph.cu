@@ -43,7 +43,7 @@ __device__ __forceinline__ double warp_max(double v) {
 }
 
 // ---- inclusive scan of row sizes into indptr[1..n] -------------------------
-static int scan_rows(int32_t* indptr, int64_t n, cudaStream_t st) {
+int scan_rows(int32_t* indptr, int64_t n, cudaStream_t st) {
   // indptr[0] = 0 and indptr[1..n] hold row sizes on entry
   if (n == 0) return GSP_OK;
   size_t bytes = 0;
@@ -151,18 +151,19 @@ __global__ void transpose_unpack_kernel(int64_t nnz, const uint64_t* __restrict_
 }
 
 template <typename T>
-static int csr_transpose(int64_t n, int64_t nnz, const int32_t* indptr, const int32_t* indices,
-                         const T* data, int32_t* t_indptr, int32_t* t_indices, T* t_data,
-                         cudaStream_t st) {
-  GSP_CUDA(cudaMemsetAsync(t_indptr, 0, sizeof(int32_t) * (n + 1), st));
-  if (n == 0 || nnz == 0) return GSP_OK;
+int csr_transpose(int64_t n_rows, int64_t n_cols, int64_t nnz, const int32_t* indptr,
+                  const int32_t* indices, const T* data, int32_t* t_indptr, int32_t* t_indices,
+                  T* t_data, cudaStream_t st) {
+  GSP_CUDA(cudaMemsetAsync(t_indptr, 0, sizeof(int32_t) * (n_cols + 1), st));
+  if (n_rows == 0 || n_cols == 0 || nnz == 0) return GSP_OK;
   uint64_t *keys_in = nullptr, *keys_out = nullptr;
   GSP_CUDA(cudaMallocAsync((void**)&keys_in, sizeof(uint64_t) * nnz, st));
   GSP_CUDA(cudaMallocAsync((void**)&keys_out, sizeof(uint64_t) * nnz, st));
-  transpose_keys_kernel<T><<<row_blocks(n), kRowThreads, 0, st>>>(n, indptr, indices, keys_in,
-                                                                   t_indptr);
+  transpose_keys_kernel<T><<<row_blocks(n_rows), kRowThreads, 0, st>>>(n_rows, indptr, indices,
+                                                                        keys_in, t_indptr);
+  // keys are (col << 32) | row: the sort covers the low 32 bits and enough high bits for n_cols
   int bits = 33;
-  while ((int64_t(1) << (bits - 32)) < n && bits < 64) ++bits;
+  while ((int64_t(1) << (bits - 32)) < n_cols && bits < 64) ++bits;
   size_t bytes = 0;
   cub::DeviceRadixSort::SortPairs(nullptr, bytes, keys_in, keys_out, data, t_data, (int)nnz, 0,
                                   bits, st);
@@ -178,8 +179,12 @@ static int csr_transpose(int64_t n, int64_t nnz, const int32_t* indptr, const in
   cudaFreeAsync(keys_in, st);
   cudaFreeAsync(keys_out, st);
   if (e != cudaSuccess) return check_cuda(e, "csr_transpose");
-  return scan_rows(t_indptr, n, st);
+  return scan_rows(t_indptr, n_cols, st);
 }
+template int csr_transpose<float>(int64_t, int64_t, int64_t, const int32_t*, const int32_t*,
+                                  const float*, int32_t*, int32_t*, float*, cudaStream_t);
+template int csr_transpose<double>(int64_t, int64_t, int64_t, const int32_t*, const int32_t*,
+                                   const double*, int32_t*, int32_t*, double*, cudaStream_t);
 
 // ---- COO -> canonical CSR (sparse.csr_matrix(coo): duplicates summed, rows sorted) ----
 __global__ void coo_keys_kernel(int64_t nnz, const int32_t* __restrict__ rows,
@@ -546,7 +551,7 @@ template int move_rows<double>(bool, int64_t, const int64_t*, const double*, int
                               const int32_t* indices, const T* data, int32_t* t_indptr,         \
                               int32_t* t_indices, T* t_data, void* stream) {                    \
     GSP_REQUIRE(nnz < (int64_t(1) << 31), "nnz must fit int32");                                \
-    return gsp::csr_transpose<T>(n, nnz, indptr, indices, data, t_indptr, t_indices, t_data,    \
+    return gsp::csr_transpose<T>(n, n, nnz, indptr, indices, data, t_indptr, t_indices, t_data, \
                                  gsp::as_stream(stream));                                       \
   }                                                                                             \
   int gsp_coo_to_csr_##SUF(int64_t n, int64_t nnz, const int32_t* rows, const int32_t* cols,     \

@@ -4,7 +4,8 @@ This is what ``Graph.W`` and ``Graph.L`` are in this engine (the reference
 holds ``scipy.sparse.csr_matrix`` objects, graph.py:109,620).  It offers the
 small read-only surface the filtering path and its callers use: ``shape``,
 ``nnz``, ``dot``, ``toarray``, ``diagonal``, plus ``to_scipy`` to leave the
-device.
+device.  ``DifferentialOperator`` holds ``Graph.D`` (the reference's CSC
+matrix, difference.py) in the two layouts its gradient and divergence walk.
 """
 import numpy as np
 
@@ -95,5 +96,88 @@ class DeviceCSR:
                          nat.stream_ptr(self.device))
         y = y.reshape((self.shape[0],) + tuple(xt.shape[1:]))
         return y.cpu().numpy() if host else y
+
+    __matmul__ = dot
+
+
+class DifferentialOperator:
+    """The N x Ne differential operator ``G.D`` (difference.py), held in HBM in two layouts.
+
+    The edge-major layout is SciPy's CSC arrays of D (``d_indptr`` over edges, vertex indices,
+    values), which is what ``grad`` walks; the vertex-major layout is D as CSR (edge ids
+    ascending in a row), which is what ``div`` walks.  ``to_scipy()`` returns the reference's
+    ``csc_matrix``; ``dot(y)`` is ``div`` and ``T.dot(x)`` is ``grad``, both on the exact-order
+    kernels of csrc/diffop.cu (results equal SciPy's on the same D bit for bit).  Not a
+    :class:`DeviceCSR`: D is rectangular and Ne < N happens.
+    """
+
+    def __init__(self, shape, d_indptr, d_indices, d_data, v_indptr, v_indices, v_data):
+        self.shape = (int(shape[0]), int(shape[1]))
+        self.d_indptr, self.d_indices, self.d_data = d_indptr, d_indices, d_data
+        self.v_indptr, self.v_indices, self.v_data = v_indptr, v_indices, v_data
+        self.T = _TransposedOperator(self)
+
+    @property
+    def nnz(self):
+        return int(self.d_indices.numel())
+
+    @property
+    def dtype(self):
+        return self.d_data.dtype
+
+    @property
+    def device(self):
+        return self.d_data.device
+
+    def __repr__(self):
+        return "<DifferentialOperator {}x{}, nnz={}, {}, {}>".format(
+            self.shape[0], self.shape[1], self.nnz, self.dtype, self.device)
+
+    def to_scipy(self):
+        from scipy import sparse
+        return sparse.csc_matrix((self.d_data.cpu().numpy(), self.d_indices.cpu().numpy(),
+                                  self.d_indptr.cpu().numpy()), shape=self.shape)
+
+    def toarray(self):
+        return self.to_scipy().toarray()
+
+    def dot(self, y):
+        """``D @ y`` (the divergence) for an edge vector or an (Ne, nsig) block."""
+        return self._product("gsp_div_", self.shape[1], self.shape[0], self.v_indptr,
+                             self.v_indices, self.v_data, y)
+
+    __matmul__ = dot
+
+    def _product(self, fn, n_in, n_out, indptr, indices, data, x):
+        torch = nat.require_cuda()
+        host = not torch.is_tensor(x)
+        xt = torch.as_tensor(np.asarray(x) if host else x).to(device=self.device, dtype=self.dtype)
+        if xt.ndim == 0 or xt.shape[0] != n_in:
+            raise ValueError("dimension mismatch")
+        nsig = int(np.prod(xt.shape[1:], dtype=np.int64))
+        flat = xt.reshape(n_in, nsig).contiguous()
+        out = torch.empty((n_out, nsig), dtype=self.dtype, device=self.device)
+        if out.numel():
+            with torch.cuda.device(self.device):
+                nat.call(fn + nat.suffix(self.dtype), nat.i64(n_out), indptr, indices, data, flat,
+                         nat.i64(nsig), out, nat.stream_ptr(self.device))
+        out = out.reshape((n_out,) + tuple(xt.shape[1:]))
+        return out.cpu().numpy() if host else out
+
+
+class _TransposedOperator:
+    """``D.T``: its ``dot(x)`` is the gradient (D^T x), over the edge-major layout."""
+
+    def __init__(self, D):
+        self._D = D
+
+    @property
+    def shape(self):
+        return (self._D.shape[1], self._D.shape[0])
+
+    def dot(self, x):
+        D = self._D
+        return D._product("gsp_grad_", D.shape[0], D.shape[1], D.d_indptr, D.d_indices,
+                          D.d_data, x)
 
     __matmul__ = dot

@@ -3,18 +3,21 @@
 Mirror of the part of ``pygsp.graphs.Graph`` that the Chebyshev filtering path
 uses (pygsp/graphs/graph.py:98-176 constructor, :510-630 compute_laplacian,
 :632-640 _check_signal, :729-838 d / dw, :840-960 lmax / estimate_lmax /
-_get_upper_bound, :368-405 is_directed).  Same constructor signature, same
-attributes, same exceptions and log messages; the adjacency, the Laplacian and
-every vector derived from them live on the GPU and are produced by the kernels
-of ``libgspb200`` (csrc/graph.cu, csrc/lanczos.cu).  Out of scope here, as in
-SURVEY.md section 2: Fourier basis, differential operator, plotting, IO.
+_get_upper_bound, :368-405 is_directed) and of its vertex calculus
+(graph.py:642-704 dirichlet_energy, :962-1029 get_edge_list, difference.py
+D / compute_differential_operator / grad / div).  Same constructor signature,
+same attributes, same exceptions and log messages; the adjacency, the
+Laplacian, the differential operator and every vector derived from them live
+on the GPU and are produced by the kernels of ``libgspb200`` (csrc/graph.cu,
+csrc/lanczos.cu, csrc/diffop.cu).  Out of scope here, as in SURVEY.md
+section 2: Fourier basis, plotting, IO.
 """
 import numpy as np
 from scipy import sparse
 
 from .. import _native as nat
 from .. import utils
-from .csr import DeviceCSR
+from .csr import DeviceCSR, DifferentialOperator
 
 _LAP = {"combinatorial": 0, "normalized": 1}
 
@@ -110,6 +113,8 @@ class Graph:
         self._lmax = None
         self._lmax_method = None
         self._lanczos_steps = None
+        self._edges = None
+        self._D = None
 
         self.lap_type = lap_type
         self.compute_laplacian(lap_type)
@@ -280,6 +285,7 @@ class Graph:
             # None (SURVEY.md 3.5); both are reset in this implementation.
             self._lmax = None
             self._lmax_method = None
+            self._D = None
         self.lap_type = lap_type
 
         torch = nat.require_cuda()
@@ -304,6 +310,114 @@ class Graph:
             raise ValueError("First dimension must be the number of vertices "
                              "G.N = {}, got {}.".format(self.N, tuple(s.shape)))
         return s
+
+    def dirichlet_energy(self, x):
+        r"""Dirichlet energy x^T L x of a vertex signal (graph.py:642-704).
+
+        L x runs on the SpMV / SpMM kernel.  A vector gives a scalar, an (N, nsig) block the
+        (nsig, nsig) matrix x^T L x; NumPy in gives NumPy out, a CUDA tensor gives a tensor.
+        """
+        torch = nat.require_cuda()
+        x = self._check_signal(x)
+        Lx = self.L.dot(x)
+        if torch.is_tensor(Lx):
+            x = x.to(device=self.device, dtype=self.dtype)
+            return torch.dot(x, Lx) if x.ndim == 1 else x.T @ Lx
+        return np.asarray(x, dtype=Lx.dtype).T.dot(Lx)
+
+    # ------------------------------------------------------- differential operator
+    def _edge_list(self):
+        """Device (sources, targets, weights) of get_edge_list (cached: W is immutable)."""
+        if self._edges is None:
+            torch = nat.require_cuda()
+            W, n = self._adjacency, self.n_vertices
+            directed = nat.i32(self.is_directed())
+            ptr = torch.empty(n + 1, dtype=torch.int32, device=self.device)
+            with torch.cuda.device(self.device):
+                nat.call("gsp_edge_list_count", nat.i64(n), W.indptr, W.indices, directed, ptr,
+                         self._stream())
+            ne = int(ptr[-1].item())
+            sources = torch.empty(ne, dtype=torch.int32, device=self.device)
+            targets = torch.empty(ne, dtype=torch.int32, device=self.device)
+            weights = torch.empty(ne, dtype=self.dtype, device=self.device)
+            self._call("gsp_edge_list_fill", nat.i64(n), W.indptr, W.indices, W.data, directed,
+                       ptr, sources, targets, weights)
+            self._edges = (sources, targets, weights)
+        return self._edges
+
+    def get_edge_list(self):
+        r"""Edge list (sources, targets, weights) of W (graph.py:962-1029).
+
+        A directed graph gives every stored entry of W in row-major order, an undirected one
+        the upper triangle (diagonal included), so that sources <= targets.  Sources and
+        targets are int32 NumPy arrays, weights are in the graph's dtype.
+        """
+        sources, targets, weights = self._edge_list()
+        assert self.n_edges == sources.numel() == targets.numel() == weights.numel()
+        return sources.cpu().numpy(), targets.cpu().numpy(), weights.cpu().numpy()
+
+    @property
+    def D(self):
+        r"""Differential operator (a :class:`DifferentialOperator`, computed lazily)."""
+        if self._D is None:
+            self.logger.warning("The differential operator G.D is not available, we need to "
+                                "compute it. Explicitly call "
+                                "G.compute_differential_operator() once beforehand to "
+                                "suppress the warning.")
+            self.compute_differential_operator()
+        return self._D
+
+    def compute_differential_operator(self):
+        r"""Compute the differential operator D, L = D D^T (difference.py; cached as G.D).
+
+        Column k of the N x Ne matrix D (edge k = (s, t) of :meth:`get_edge_list`) holds
+        -sqrt(W[s, t]) at s and +sqrt(W[s, t]) at t (combinatorial), or -sqrt(W[s, t] / dw[s])
+        and +sqrt(W[s, t] / dw[t]) (normalized), both divided by sqrt(2) for a directed graph;
+        a self-loop's column is empty.
+        """
+        torch = nat.require_cuda()
+        sources, targets, weights = self._edge_list()
+        n, ne = self.n_vertices, self.n_edges
+        d_indptr = torch.empty(ne + 1, dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            nat.call("gsp_diffop_count", nat.i64(ne), sources, targets, d_indptr, self._stream())
+        nnz = int(d_indptr[-1].item())
+        d_indices = torch.empty(nnz, dtype=torch.int32, device=self.device)
+        d_data = torch.empty(nnz, dtype=self.dtype, device=self.device)
+        v_indptr = torch.empty(n + 1, dtype=torch.int32, device=self.device)
+        v_indices = torch.empty(nnz, dtype=torch.int32, device=self.device)
+        v_data = torch.empty(nnz, dtype=self.dtype, device=self.device)
+        self._call("gsp_diffop_fill", nat.i64(n), nat.i64(ne), nat.i64(nnz), sources, targets,
+                   weights, self._degrees()[0], nat.i32(_LAP[self.lap_type]),
+                   nat.i32(self.is_directed()), d_indptr, d_indices, d_data, v_indptr, v_indices,
+                   v_data)
+        self._D = DifferentialOperator((n, ne), d_indptr, d_indices, d_data, v_indptr,
+                                       v_indices, v_data)
+
+    def grad(self, x):
+        r"""Gradient D^T x of a vertex signal (difference.py grad).
+
+        x is (N,) or (N, nsig); the result is (Ne,) or (Ne, nsig) in the graph's dtype, equal
+        bit for bit to SciPy's ``G.D.to_scipy().T.dot(x)``.  NumPy in gives NumPy out, a CUDA
+        tensor gives a tensor.
+        """
+        x = self._check_signal(x)
+        return self.D.T.dot(x)
+
+    def div(self, y):
+        r"""Divergence D y of an edge signal (difference.py div).
+
+        y is (Ne,) or (Ne, nsig); the result is (N,) or (N, nsig) in the graph's dtype, equal
+        bit for bit to SciPy's ``G.D.to_scipy().dot(y)``.  NumPy in gives NumPy out, a CUDA
+        tensor gives a tensor.
+        """
+        torch = nat.require_cuda()
+        if not torch.is_tensor(y):
+            y = np.asanyarray(y)
+        if y.shape[0] != self.Ne:
+            raise ValueError("First dimension must be the number of edges "
+                             "G.Ne = {}, got {}.".format(self.Ne, tuple(y.shape)))
+        return self.D.dot(y)
 
     # ------------------------------------------------------------------------ lmax
     @property
